@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- batched BFGS step! throughput (BASELINE.json configs[1]) + n=16384 step! roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (N=1): 1,000,000 independent extended-Rosenbrock problems, n=16, x0 = 4u-2 with u from
 the reference's PCG (legacy/PCG.jl, seed 2024+rank), initial step 1.0.  One "step" = one step!
@@ -24,6 +24,10 @@ Numbers on the JSON line
   riesz_gd  config 5 with its FP64-pipe roofline
   cpu_baseline  the CPU oracle (a port of the reference: the reference itself is commented-out
             Julia and no Julia exists here) on all host threads, bounded sample
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step! left in its batch (see dump_outputs) as
+DIR/<field>.npy.  The inputs depend only on the arguments, so two builds can be compared output for output.
+The benchmark writes nothing into the source tree: the CPU arm's native oracle build goes to a temporary directory.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree (it may be read-only)
 
 N_SMALL = 16
 BATCH = 1_000_000
@@ -49,6 +54,8 @@ SHARDED_CHECK_N = 8192
 STEPS_PER_BATCH = 25            # timed step! calls per batch (a batch converges within ~100 calls: see device_timed)
 METRIC = "batched BFGS problem-steps/s (1M x n=16)"
 UNIT = "problem-steps/s"
+DUMP_PROBLEMS = 65536           # --dump-outputs: problems of the last timed batch written out (a fixed, seeded sample)
+DUMP_SEED = 0
 
 
 def bytes_by_kind(n, lazy=True):
@@ -102,6 +109,21 @@ def oracle_mod():
 def x0_batch(gen, batch, seed):
     """gen: anything with pcg_fill(count, seed) -- the product package in the GPU arm, the oracle in the reference arm"""
     return (4.0 * gen.pcg_fill(batch * N_SMALL, seed) - 2.0).reshape(batch, N_SMALL)
+
+
+def dump_outputs(opt, out_dir):
+    """--dump-outputs DIR: the fields a caller of step! reads, as the last timed step! left them in its batch, for the
+    same DUMP_PROBLEMS problems of the batch in every run (their indices in problem_index.npy), one float64 .npy per
+    field, 28 MB in all.  Fields with n = 16 values per problem have shape (DUMP_PROBLEMS, 16), the others (DUMP_PROBLEMS,)."""
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(BATCH, DUMP_PROBLEMS, replace=False))
+    fields = {"current_point": opt.current_point, "current_gradient": opt.current_gradient,
+              "next_step_direction": opt.next_step_direction, "current_objective_value": opt.current_objective_value,
+              "last_step_length": opt.last_step_length, "last_step_type": opt.last_step_type,
+              "iteration_count": opt.iteration_count, "has_converged": opt.has_converged}
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "problem_index.npy"), rows.astype(np.float64))
+    for name, a in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a)[rows].astype(np.float64))
 
 
 class ClockSampler:
@@ -350,12 +372,13 @@ def run_gpu(args):
         o.set_stream(stream.cuda_stream)
         return o
 
-    def device_timed(x0_list):
+    def device_timed(x0_list, dump_dir=None):
         """K back-to-back step! launches after W warm-up steps per batch.  A batch of this workload converges within ~100
         step! calls, so K > STEPS_PER_BATCH launches walk through ceil(K / STEPS_PER_BATCH) independent batches of the same
         synthetic workload (each constructed and warmed up before the clock starts): every timed launch is a step! in
         the regime the metric is quoted on, however long the timed region.  Returns (ms max over ranks, kind counts of
-        this rank summed over the batches, clock sampler)."""
+        this rank summed over the batches, clock sampler).  With dump_dir, the batch of the last timed launch is written
+        there after the clock stops (dump_outputs)."""
         opts = [make(x) for x in x0_list]
         for o in opts:
             o.step(W)
@@ -370,6 +393,8 @@ def run_gpu(args):
             ev1.record(stream)
             barrier()
             ms = ev0.elapsed_time(ev1)
+        if dump_dir is not None:
+            dump_outputs(opts[(K - 1) // STEPS_PER_BATCH], dump_dir)
         kinds = {}
         for o in opts:
             for k, v in o.step_kind_counts().items():
@@ -437,7 +462,7 @@ def run_gpu(args):
     x0_hosts = [torch.from_numpy(x0_batch(dz, BATCH, 2024 + rank + 1000 * b)).pin_memory().numpy() for b in range(nbatches)]
     x0_host = x0_hosts[0]
     x0 = x0_host
-    ms, kinds, clk = device_timed(x0_hosts)
+    ms, kinds, clk = device_timed(x0_hosts, dump_dir=args.dump_outputs if rank == 0 else None)
     launches += K
     active_steps = float(sum(kinds[k] for k in ("bfgs_read_h", "bfgs_identity_h", "gradient_descent", "terminate")))
     total_problem_steps = sum_over_ranks(active_steps)
@@ -947,7 +972,13 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="multi-rank runs: leave the ranks' CPU affinity alone (A/B)")
     ap.add_argument("--cpu-sample", type=int, default=50_000)
     ap.add_argument("--tune", action="append", default=[], help="key=value passed to dzo_set_tuning (A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<field>.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -7,6 +7,7 @@ import ctypes as C
 import importlib.util
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -46,17 +47,17 @@ NATIVE_FLAGS = "-O3 -march=native -ffp-contract=off -fno-fast-math -fopenmp -fPI
 
 def use_native_build():
     """bench.py's CPU arm: the same source compiled for THIS host's cores (-O3 -march=native, still no contraction
-    and no reassociation, so every bit stays the same -- tests/test_oracle.py asserts it).  Built where it runs (the
-    GPU box's CPU differs from the build container's); must be called before the first oracle call of the process."""
+    and no reassociation, so every bit stays the same -- tests/test_oracle.py asserts it).  Compiled at run time for the
+    host that runs it, into a temporary directory so that the source tree may be read-only; must be called before the
+    first oracle call of the process."""
     global _lib
     if _lib is not None and getattr(_lib, "_dzo_native", False):
         return NATIVE_FLAGS
-    out_dir = os.path.join(_HERE, "_build", "native")
-    out = os.path.join(out_dir, "libdzo_oracle_native.so")
-    os.makedirs(out_dir, exist_ok=True)
-    subprocess.run(["gcc"] + NATIVE_FLAGS.split() + ["-shared", "-o", out, os.path.join(_HERE, "dzo_oracle.c"), "-lm"],
-                   check=True, capture_output=True)
-    _lib = _capi.bind(C.CDLL(out), cpu=True)
+    with tempfile.TemporaryDirectory(prefix="dzo_oracle_native_") as tmp:
+        out = os.path.join(tmp, "libdzo_oracle_native.so")
+        subprocess.run(["gcc"] + NATIVE_FLAGS.split() + ["-shared", "-o", out, os.path.join(_HERE, "dzo_oracle.c"), "-lm"],
+                       check=True, capture_output=True)
+        _lib = _capi.bind(C.CDLL(out), cpu=True)      # stays mapped after the file is removed
     _lib._dzo_native = True
     return NATIVE_FLAGS
 

@@ -51,18 +51,30 @@ def test_product_library_does_not_link_the_oracle(dz):
 
 
 def test_no_gpu_means_loud_failure_not_fallback(dz):
-    """On this CPU-only box the constructor must raise DZO_ERR_NO_DEVICE (-6), never compute."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    EF = dz.ExampleFunctions
-    with pytest.raises(dz.DZOptError) as e:
-        dz.BFGSOptimizer(EF.rosenbrock_function, EF.rosenbrock_gradient_, np.zeros(2), 1.0)
-    assert e.value.code == -6
-    with pytest.raises(dz.DZOptError) as e:
-        dz.GradientDescentOptimizer(EF.rosenbrock_function, EF.rosenbrock_gradient_, dz.QuadraticLineSearch(0),
-                                    np.zeros(64), 1.0)
-    assert e.value.code == -6
+    """Without a CUDA device the constructor must raise DZO_ERR_NO_DEVICE (-6), never compute.  Runs in a child process
+    with CUDA_VISIBLE_DEVICES="", which hides every device, so the check also runs on a machine that has GPUs."""
+    import subprocess
+    import sys
+    child = "\n".join([
+        "import sys",
+        "sys.path.insert(0, %r)" % ROOT,
+        "import numpy as np",
+        "import dzopt_b200 as dz",
+        "EF = dz.ExampleFunctions",
+        "makers = [lambda: dz.BFGSOptimizer(EF.rosenbrock_function, EF.rosenbrock_gradient_, np.zeros(2), 1.0),",
+        "          lambda: dz.GradientDescentOptimizer(EF.rosenbrock_function, EF.rosenbrock_gradient_,",
+        "                                              dz.QuadraticLineSearch(0), np.zeros(64), 1.0)]",
+        "for make in makers:",
+        "    try:",
+        "        make()",
+        "        print('computed')",
+        "    except dz.DZOptError as e:",
+        "        print(e.code)",
+    ])
+    r = subprocess.run([sys.executable, "-c", child], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.split() == ["-6", "-6"], r.stdout
 
 
 def test_constructor_argument_validation(dz):
