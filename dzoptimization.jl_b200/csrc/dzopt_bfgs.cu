@@ -408,14 +408,12 @@ static int large_step_once(dzo_bfgs* o) {
         launch_warp_search(o, vw, v, false);                                            // :891-950, :873-874
         DZO_CUDA(cudaGetLastError());
         sa.v = o->dg; sa.out = o->t;                                                    // :875
-        if (o->n <= 64) warp_gemv_kernel<2, 16><<<grid, threads, 0, o->stream>>>(sa);
-        else warp_gemv_kernel<4, 8><<<grid, threads, 0, o->stream>>>(sa);
+        warp_gemv_kernel<2, 16><<<grid, threads, 0, o->stream>>>(sa);
         DZO_CUDA(cudaGetLastError());
         launch_warp_search(o, vw, v, true);                                             // :876
         DZO_CUDA(cudaGetLastError());
         sa.v = o->g; sa.out = o->d;                                                     // :878-886 + :958-960, :981
-        if (o->n <= 64) warp_update_gemv_kernel<2, 16><<<grid, threads, 0, o->stream>>>(sa);
-        else warp_update_gemv_kernel<4, 8><<<grid, threads, 0, o->stream>>>(sa);
+        warp_update_gemv_kernel<2, 16><<<grid, threads, 0, o->stream>>>(sa);
         DZO_CUDA(cudaGetLastError());
         return DZO_OK;
     }

@@ -2,12 +2,12 @@
 //
 // gemv_kernel / update_gemv_kernel (large_bfgs.cuh) give every problem of a batch its own CTA (blockIdx.z); at n = 64 that
 // CTA has 32 working threads and a shared-memory prologue per 32 KB of matrix (0.58 of the HBM peak for 16384 problems).
-// Here a lane owns RPL = 2 adjacent rows of its problem's matrix (RPL = 4 for n <= 128 is written and parity-tested but
-// measured no faster than the tiled kernels -- 0.549 vs 0.542 ms per step! call for 8192 problems of n = 128 -- and not
-// dispatched; n = 34: 0.203 -> 0.177 ms for 16384 problems, n = 64: 0.338 -> 0.307), a warp reads 512 contiguous bytes of
-// every column, the vector operands are broadcast loads, and four problems share a CTA with nothing
-// in common.  Per row the accumulation is the same strictly sequential walk over the columns (n <= 1024: a single chunk of
-// the canonical GEMV order), so the results are those of the tiled kernels bit for bit.
+// Here a lane owns RPL = 2 adjacent rows of its problem's matrix (n = 34: 0.203 -> 0.177 ms for 16384 problems, n = 64:
+// 0.338 -> 0.307), a warp reads 512 contiguous bytes of every column, the vector operands are broadcast loads, and four
+// problems share a CTA with nothing in common.  Per row the accumulation is the same strictly sequential walk over the
+// columns (n <= 1024: a single chunk of the canonical GEMV order), so the results are those of the tiled kernels bit for bit.
+// The templates take any even RPL (n <= 32 RPL), but only RPL = 2 is dispatched and tested: RPL = 4 for n <= 128 was
+// measured no faster than the tiled kernels (0.549 vs 0.542 ms per step! call for 8192 problems of n = 128).
 //
 // legacy/DZOptimization.jl:875 (t = H * dg), :878-886 (rank-2 update, exact operation order of :882-884) fused with
 // :958-960 (d = H' * g), :981 (identity_matrix! after a gradient-descent step).
