@@ -127,6 +127,7 @@ def bind(lib, cpu: bool):
         sig("gd_step_async", [H, I])
         sig("gd_sync", [H])
         sig("gd_info", [H, c_i64_p, c_i64_p, c_int_p])
+        sig("gd_riesz_info", [H, c_int_p, c_int_p, c_int_p, c_int_p, c_int_p, c_int_p])
         sig("gd_get_evaluation_count", [H, c_i64_p])
         sig("gd_get_phase_log", [H, C.POINTER(C.c_uint64), I64, c_i64_p])
         sig("identity", [I64, c_double_p, I])

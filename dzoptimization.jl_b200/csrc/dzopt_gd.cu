@@ -385,6 +385,19 @@ int dzo_gd_info(dzo_gd* o, int64_t* n, int64_t* batch, int* order) {
     if (order) *order = o->small ? DZO_ORDER_SEQUENTIAL : (o->gridgd ? DZO_ORDER_TREE_BLOCKED : DZO_ORDER_TREE);
     return DZO_OK;
 }
+int dzo_gd_riesz_info(dzo_gd* o, int* threads_per_cta, int* ctas, int* energy_lanes_per_row, int* paired_probes,
+                      int* gradient_tiles, int* flag_barrier) {
+    if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");
+    if (o->small || o->objective != DZO_OBJ_RIESZ)
+        return fail(DZO_ERR_UNSUPPORTED, "riesz info: one-problem Riesz handles (n > %d) only", DZO_SMALL_N_MAX);
+    if (threads_per_cta) *threads_per_cta = o->nt;
+    if (ctas) *ctas = o->grid;
+    if (energy_lanes_per_row) *energy_lanes_per_row = o->esplit;
+    if (paired_probes) *paired_probes = (o->espec != 0 && o->esplit != 2) ? 1 : 0;   // what line_search uses
+    if (gradient_tiles) *gradient_tiles = o->gvariant;
+    if (flag_barrier) *flag_barrier = (o->bar != nullptr) ? 1 : 0;
+    return DZO_OK;
+}
 
 }  // extern "C"
 
