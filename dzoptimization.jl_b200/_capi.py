@@ -115,6 +115,7 @@ def bind(lib, cpu: bool):
         sig("bfgs_get_step_log", [H, c_i64_p, c_u8_p])
         sig("bfgs_gather_mode", [H, c_int_p])
         sig("bfgs_get_step_kind_counts", [H, c_i64_p, I])
+        sig("bfgs_batched_layout", [H, c_int_p, c_int_p])
         sig("bfgs_mirror_fields", [H, c_double_p, c_u8_p])
         sig("lbfgs_set_stream", [H, C.c_void_p])
         sig("lbfgs_step_async", [H, I])

@@ -25,10 +25,26 @@ struct BatchedArgs {
     int ksteps;
     int prefetch_rounds;  // hybrid kernel: phase-2 rounds whose H tiles are pulled into L2 ahead of use
     int tile;             // hybrid kernel: problems per warp (0 or 32: a full warp; smaller for batches of a few waves)
-    unsigned char* hid;          // optional (may be null): hid[p] != 0 <=> H of problem p is the identity and its copy in
-                                 //   HBM is stale (identity_matrix! :981 / :781-783 not materialised; hybrid kernel only)
+    unsigned char* flags;        // Rosenbrock handles: per-problem state byte, BF_* bits below
+    int lazy;                    // keep H = I implicit (BF_IDENT)
+    int derived;                 // derived layout: a move stores x into the other point buffer (x / g, BF_PARITY) and no
+                                 //   g, dx or dg; g = rosenbrock_gradient!(x), dx, dg are recomputed from the two points
     unsigned long long* stats;   // optional (may be null): HK_COUNT running step-kind counters
 };
+// flags[p]: BF_IDENT     H of problem p is the identity and its copy in HBM is stale (identity_matrix! :981 / :781-783
+//                        not materialised)
+//           BF_PARITY    derived layout: the current point is in g (set) or x (clear); the other buffer holds the previous one
+//           BF_EXPLICIT  derived layout: delta_point / delta_gradient are the dx / dg arrays (constructor, set_state), not
+//                        the differences of the two points
+enum : unsigned { BF_IDENT = 1u, BF_PARITY = 2u, BF_EXPLICIT = 4u };
+
+// rosenbrock_gradient! of one consecutive pair (legacy/ExampleFunctions.jl): the expression, hence the bits, of
+// RosenbrockSmall::grad and of the step kernel, so the derived layout can recompute g wherever it needs it
+DZO_DEVINL double2 rosen_pair_grad(double xe, double xo) {
+    const double t1 = 1 - xe;
+    const double t2 = xo - xe * xe;
+    return make_double2(-2 * t1 - 400 * xe * t2, 200 * t2);
+}
 
 constexpr int kBatchedThreads = 256;
 constexpr int kBcBufs = 5;  // 2 rotating reduction buffers + 3 vector broadcast buffers
@@ -197,11 +213,11 @@ static __global__ void __launch_bounds__(kBatchedThreads) bfgs_batched_init_kern
     const double f0 = Obj::eval(G, x);                              // :772
     const double g = Obj::grad(G, x);                               // :775-776
     if (G.act) {
-        A.g[p * n + G.r] = g;
+        if (!A.derived) A.g[p * n + G.r] = g;
         A.d[p * n + G.r] = g;                                       // :784 next_step_direction = copy(gradient)
         A.dx[p * n + G.r] = 0.0;                                    // :777
         A.dg[p * n + G.r] = 0.0;                                    // :778
-        if (!A.hid) {
+        if (!A.lazy) {
             double* Hp = A.H + p * n * n;                           // :781-783 identity_matrix!
             for (int j = 0; j < n; ++j) Hp[G.r + j * n] = (j == G.r) ? 1.0 : 0.0;
         }
@@ -212,7 +228,7 @@ static __global__ void __launch_bounds__(kBatchedThreads) bfgs_batched_init_kern
         A.iter[p] = 0;                                              // :767
         A.type[p] = DZO_STEP_NULL;                                  // :780
         A.term[p] = 0;                                              // :768
-        if (A.hid) A.hid[p] = 1;                                    // H = I, kept implicit (batched_hybrid.cuh)
+        A.flags[p] = (A.lazy ? BF_IDENT : 0u) | BF_EXPLICIT;        // H = I kept implicit (batched_hybrid.cuh); x in x
     }
 }
 
@@ -248,13 +264,13 @@ static __global__ void __launch_bounds__(kBatchedThreads) bfgs_batched_restore_k
     if (G.act)
         for (int j = 0; j < n; ++j) d += Hp[G.r + j * n] * v0[j];   // mul!(d, H, g), row sum j ascending
     if (G.act) {
-        A.g[p * n + G.r] = g;
+        if (!A.derived) A.g[p * n + G.r] = g;
         A.d[p * n + G.r] = d;
     }
     if (G.r == 0) {
         A.f[p] = f0;
         A.term[p] = 0;
-        if (A.hid) A.hid[p] = 0;                                    // the caller's H is in HBM
+        A.flags[p] = BF_EXPLICIT;                                   // the caller's H, x, dx and dg are in HBM
     }
 }
 

@@ -8,7 +8,8 @@
 //            different searches share the expensive code), the BFGS / GD / terminate decision, overlap.
 //            The vectors live in a per-warp shared-memory tile [32 problems][n + 2] (16-byte aligned rows).
 //   phase 2  NP LANES PER PROBLEM (NP = n rounded up to a power of two), uniform control flow: lane r recomputes element r
-//            of x, g, dx, dg (bit-identical elementwise formulas) and stores them coalesced, streams ROW r of the
+//            of x, g, dx, dg (bit-identical elementwise formulas) and stores them coalesced (the derived layout stores
+//            only x, into the other point buffer), streams ROW r of the
 //            inverse Hessian from HBM into registers with coalesced loads (for a fixed column the lanes of a problem
 //            read n consecutive doubles; two register tiles ping-pong so the next round's rows are in flight while the
 //            current round computes; tiles further ahead are pulled into L2 with prefetch.global.L2), t = H*dg,
@@ -16,7 +17,7 @@
 //
 // What round 2 changed (each step A/B'd inside one gpurun call, profiles/README.md; 0.89 -> 0.74 ms per 1M-problem launch):
 //   * LAZY identity: identity_matrix! (:981) after a gradient-descent step is not written to HBM; a per-problem byte
-//     `hid` says "H is the identity, the copy in HBM is stale".  The next BFGS-type step builds its rows of I in registers
+//     `flags` bit BF_IDENT says "H is the identity, the copy in HBM is stale".  The next BFGS-type step builds its rows of I in registers
 //     instead of loading them (the same arithmetic on the same values), the constructor writes no H at all, and
 //     dzo_bfgs_get_inverse_hessian materialises I for the caller.  A GD-type step moves 1.1 KB instead of 3.1 KB and a
 //     BFGS-type step after it 3.1 KB instead of 5.2 KB (n = 16).
@@ -31,6 +32,11 @@
 //   Measured and rejected: both line searches side by side in one thread (0.95 ms: register spills in the probe loop, and
 //   max(probes) per iteration of two searches costs more issue slots than the shared state machine); persistent CTAs with
 //   tiles handed to warps through a counter (0.80 ms: 2.0 instead of 0.3 no-instruction stall cycles per issue).
+// What round 3 changed: the DERIVED layout (Tuning::batched_derived).  g is always rosenbrock_gradient!(x) and dx, dg are
+//   differences of two points, so a move writes its new x into the second point buffer (the old x stays in the first)
+//   and stores no g, dx or dg; the tile's G rows are recomputed from X after staging, and the getters recompute the
+//   fields bit for bit from the two points (flags bits BF_PARITY / BF_EXPLICIT, batched_bfgs.cuh).  512 B less per
+//   moving problem-step at n = 16 (DESIGN.md section 3).
 //
 // legacy/DZOptimization.jl:891-994 (step!), :864-889 (update_inverse_hessian!), :49-216 (line search).
 #pragma once
@@ -63,8 +69,9 @@ struct HybridCfg {
 template <int N>
 struct HybridSmem {
     using C = HybridCfg<N>;
-    alignas(16) double X[32][C::STRIDE];       // current_point          -> after phase 1: delta_gradient
-    alignas(16) double G[32][C::STRIDE];       // current_gradient       -> after phase 1: new gradient
+    alignas(16) double X[32][C::STRIDE];       // current_point          -> in phase 2: delta_gradient
+    alignas(16) double G[32][C::STRIDE];       // current_gradient (staged, or recomputed from X by the derived layout)
+                                               //                        -> in phase 2: new gradient
     alignas(16) double D[32][C::STRIDE];       // next_step_direction    -> after phase 1: step_direction / overlap
     alignas(16) double T[C::PPR][C::NP];       // scratch = H * delta_gradient of the problems of the current round
     alignas(16) double P[C::PPR][C::NP];       // products for the sequential dot of :876
@@ -72,7 +79,7 @@ struct HybridSmem {
 // The two spare doubles of the three rows of problem q carry what phase 1 hands to phase 2:
 //   X[q][SLOT]    lane q < HK_COUNT: running step-kind counter q of this warp     X[q][SLOT+1]  alpha = -step length (:945/:973)
 //   G[q][SLOT]    alpha * overlap  (first operand of :876)                         G[q][SLOT+1]  1 / overlap          (:874)
-//   D[q][SLOT]    low word: step kind | where H comes from << 8                    D[q][SLOT+1]  (free)
+//   D[q][SLOT]    low word: step kind | where H comes from << 8 | x goes to g << 16  D[q][SLOT+1]  (free)
 
 enum : int { HS_INIT = 0, HS_EXPAND = 1, HS_SHRINK = 2, HS_QUAD = 3, HS_DONE = 4 };
 
@@ -173,8 +180,10 @@ DZO_DEVINL void hs_probe(const double* X, const double* Dir, double a, double ar
 enum : int { HK_BFGS_READ = 0, HK_BFGS_IDENT = 1, HK_GD = 2, HK_TERMINATE = 3, HK_IDLE = 4, HK_IDLE_WARP = 5, HK_COUNT = 6 };
 
 // VTILE: problems per warp taken from A.tile (small batches) instead of the compile-time 32 -- a second instantiation
-// because the run-time tile costs the n = 16 kernel two more spilled registers (0.699 -> 0.706 ms per 1 M-problem launch)
-template <int N, bool VTILE>
+// because the run-time tile costs the n = 16 kernel two more spilled registers (0.699 -> 0.706 ms per 1 M-problem launch).
+// DERIVED: the layout of BatchedArgs::derived, a template parameter for the same reason (run-time branches on it cost
+// the n = 16 full-tile kernel 8 more bytes of spill stores).
+template <int N, bool VTILE, bool DERIVED>
 __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfgs_batched_hybrid_kernel(BatchedArgs A) {
     using C = HybridCfg<N>;
     static_assert(HK_COUNT <= 32, "one counter per lane");
@@ -192,22 +201,26 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
     const long long p = p0 + lane;
     const bool valid = VTILE ? (lane < tile && p < A.batch) : (p < A.batch);
     const int nprob = (int)((A.batch - p0 < tile) ? (A.batch - p0) : tile);
-    const bool lazy = (A.hid != nullptr);
+    const bool lazy = A.lazy != 0;
+    constexpr bool derived = DERIVED;
 
-    // A tile starts cold: everything it needs first is requested at once -- the three vectors as 16-byte asynchronous
-    // copies straight into the shared tile (no registers held), flags and scalars as ordinary loads in flight beside them.
-    auto stage_vectors = [&]() {
+    // A tile starts cold: everything it needs first is requested at once -- the vectors as 16-byte asynchronous copies
+    // straight into the shared tile (no registers held), flags and scalars as ordinary loads in flight beside them.
+    // The derived layout copies no g (filled from X below) and takes x of problem q from g when bit q of `odd` is set;
+    // `odd` is a ballot of the flags bytes, so its first copies wait for the flags load (one dependent round trip per
+    // tile; not measured on its own -- the layout A/B in profiles/ includes it).
+    auto stage_vectors = [&](unsigned odd) {
         for (int e2 = lane; e2 < nprob * (N / 2); e2 += 32) {
             const int q = (2 * e2) / N, i = 2 * e2 - q * N;
-            cp_async16(&S.X[q][i], A.x + p0 * N + 2 * e2);
-            cp_async16(&S.G[q][i], A.g + p0 * N + 2 * e2);
+            cp_async16(&S.X[q][i], (((odd >> q) & 1u) ? A.g : A.x) + p0 * N + 2 * e2);
+            if (!derived) cp_async16(&S.G[q][i], A.g + p0 * N + 2 * e2);
             cp_async16(&S.D[q][i], A.d + p0 * N + 2 * e2);
         }
         cp_async_commit();
     };
-    stage_vectors();
+    unsigned fl = (valid && (lazy || derived)) ? A.flags[p] : 0u;   // BF_* (batched_bfgs.cuh)
+    stage_vectors(derived ? __ballot_sync(FULL, (fl & BF_PARITY) != 0u) : 0u);
     bool term = valid ? (A.term[p] != 0) : true;
-    bool ident = (lazy && valid) ? (A.hid[p] != 0) : false;    // H == I and the copy in HBM is stale
     bool moved_any = false;
     double& cnt_slot = S.X[lane][SLOT];                        // lane k < HK_COUNT: running counter k (exact below 2^53)
     cnt_slot = 0.0;
@@ -223,8 +236,9 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
             // a later step of the same launch: the vectors were stored by other lanes of this warp in phase 2
             __threadfence_block();
             __syncwarp();
-            stage_vectors();
+            stage_vectors(derived ? __ballot_sync(FULL, (fl & BF_PARITY) != 0u) : 0u);
         }
+        const bool ident = lazy && (fl & BF_IDENT);    // H == I and the copy in HBM is stale
         double f0 = valid ? A.f[p] : 0.0;              // (a later step of the same launch reads back its own stores)
         double L = valid ? A.L[p] : 0.0;
         const double* X = S.X[lane];
@@ -258,6 +272,15 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
         for (int rr = 0; rr < A.prefetch_rounds; ++rr) prefetch_round(rr);
         cp_async_wait_all();
         __syncwarp();
+        if (derived) {
+            // g = rosenbrock_gradient!(x): the bits the old layout stored and staged
+            for (int e2 = lane; e2 < nprob * (N / 2); e2 += 32) {
+                const int q = (2 * e2) / N, i = 2 * e2 - q * N;
+                const double2 x2 = *reinterpret_cast<const double2*>(&S.X[q][i]);
+                *reinterpret_cast<double2*>(&S.G[q][i]) = rosen_pair_grad(x2.x, x2.y);
+            }
+            __syncwarp();
+        }
 
         // ---------------------------------------------------------------- phase 1: one thread per problem
         {
@@ -307,7 +330,7 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
             if (kind == DZO_STEP_BFGS) {
                 // overlap = dot(step_direction, delta_gradient)  :873 -- thread-local and strictly sequential.
                 // The elementwise results (x, g, dx, dg, d/overlap) are recomputed bit-identically by the
-                // phase-2 lanes, which can store them coalesced.
+                // phase-2 lanes, which store the ones the layout keeps coalesced.
 #pragma unroll
                 for (int k = 0; k < N / 2; ++k) {
                     const double xa = X[2 * k], xc = X[2 * k + 1];
@@ -345,13 +368,15 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
                     if (A.term_host) A.term_host[p] = 1;
                 }
                 const bool ident_next = (kind == DZO_STEP_BFGS) ? false : ((kind == DZO_STEP_GRADIENT_DESCENT) ? lazy : ident);
-                if (lazy && ident_next != ident) A.hid[p] = ident_next ? 1 : 0;
-                ident = ident_next;
+                unsigned fl_next = ident_next ? (fl | BF_IDENT) : (fl & ~BF_IDENT);
+                if (derived && kind != DZO_STEP_NULL) fl_next = (fl_next ^ BF_PARITY) & ~BF_EXPLICIT;   // x moves to the other buffer
+                if (fl_next != fl) A.flags[p] = (unsigned char)fl_next;
+                fl = fl_next;
             }
             S.X[lane][SLOT + 1] = alpha;
             S.G[lane][SLOT] = alpha * overlap;                                            // first operand of :876
             S.G[lane][SLOT + 1] = 1.0 / overlap;                                          // :874 inv(overlap)
-            reinterpret_cast<int*>(&S.D[lane][SLOT])[0] = kind | (hsrc << 8);
+            reinterpret_cast<int*>(&S.D[lane][SLOT])[0] = kind | (hsrc << 8) | ((derived && (fl & BF_PARITY)) ? (1 << 16) : 0);
         }
         __syncwarp();
 
@@ -364,7 +389,7 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
         auto load_rows = [&](int round, double (&row)[N], int& meta) {
             const int q = round * PPR + sub;
             meta = reinterpret_cast<const int*>(&S.D[q][SLOT])[0];
-            if (act && (meta >> 8) == 1) {
+            if (act && ((meta >> 8) & 0xff) == 1) {
                 const double* Hp = A.H + (p0 + q) * NN + r;          // H[r, j] at Hp[j*N] (column-major)
 #pragma unroll
                 for (int j = 0; j < N; ++j) row[j] = __ldcs(Hp + j * N);
@@ -385,15 +410,17 @@ __global__ void __launch_bounds__(kHybridThreads, HybridCfg<N>::CTAS_PER_SM) bfg
             const double t2_ = xod - xe * xe;
             const double gn = (r & 1) ? (200 * t2_) : (-2 * t1_ - 400 * xe * t2_);    // :948 rosenbrock_gradient!
             const double dgv = (-go) + gn;                                            // :944, :950
-            A.x[e] = xn;
-            A.g[e] = gn;
-            A.dx[e] = (-xo) + xn;                                                     // :943, :949
-            A.dg[e] = dgv;
+            ((derived && (meta >> 16)) ? A.g : A.x)[e] = xn;                          // derived: the buffer the flags now name
+            if (!derived) {
+                A.g[e] = gn;
+                A.dx[e] = (-xo) + xn;                                                 // :943, :949
+                A.dg[e] = dgv;
+            }
             double* Hp = A.H + (p0 + q) * NN + r;
             if (kcur == DZO_STEP_BFGS) {
                 // update_inverse_hessian!  :874-886 fused with mul!(d, H, g)  :958-960
                 const double ao_q = S.G[q][SLOT], inv_overlap_q = S.G[q][SLOT + 1];
-                if ((meta >> 8) == 2) {
+                if (((meta >> 8) & 0xff) == 2) {
 #pragma unroll
                     for (int j = 0; j < N; ++j) cur[j] = (j == r) ? 1.0 : 0.0;        // the rows identity_matrix! would have left
                 }
@@ -492,16 +519,23 @@ inline cudaError_t hybrid_launch(const BatchedArgs& args, cudaStream_t stream, i
     static const size_t pad = getenv("DZO_HYBRID_SMEM_PAD") ? (size_t)atoi(getenv("DZO_HYBRID_SMEM_PAD")) : 0;   // occupancy experiments
     const size_t smem = hybrid_smem<N>() + pad;
     if (!attr_set[device & 63]) {
-        cudaError_t e = cudaFuncSetAttribute(bfgs_batched_hybrid_kernel<N, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(bfgs_batched_hybrid_kernel<N, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
+        for (auto* k : {bfgs_batched_hybrid_kernel<N, false, false>, bfgs_batched_hybrid_kernel<N, true, false>,
+                        bfgs_batched_hybrid_kernel<N, false, true>, bfgs_batched_hybrid_kernel<N, true, true>}) {
+            const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+        }
         attr_set[device & 63] = true;
     }
     const bool vtile = (args.tile > 0 && args.tile < 32);
     const int tile = vtile ? args.tile : 32;
     const unsigned grid = (unsigned)((args.batch + (long long)tile * kHybridWarps - 1) / ((long long)tile * kHybridWarps));
-    if (vtile) bfgs_batched_hybrid_kernel<N, true><<<grid, kHybridThreads, smem, stream>>>(args);
-    else bfgs_batched_hybrid_kernel<N, false><<<grid, kHybridThreads, smem, stream>>>(args);
+    if (args.derived) {
+        if (vtile) bfgs_batched_hybrid_kernel<N, true, true><<<grid, kHybridThreads, smem, stream>>>(args);
+        else bfgs_batched_hybrid_kernel<N, false, true><<<grid, kHybridThreads, smem, stream>>>(args);
+    } else {
+        if (vtile) bfgs_batched_hybrid_kernel<N, true, false><<<grid, kHybridThreads, smem, stream>>>(args);
+        else bfgs_batched_hybrid_kernel<N, false, false><<<grid, kHybridThreads, smem, stream>>>(args);
+    }
     return cudaGetLastError();
 }
 cudaError_t hybrid_launch_n2_16(int n, const BatchedArgs& args, cudaStream_t stream, int device);    // batched_hybrid_tu_a.cu

@@ -102,7 +102,9 @@ struct dzo_bfgs {
     double* f_host = nullptr;            // dzo_bfgs_mirror_fields: page-locked host mirrors written by the step kernels
     unsigned char* term_host = nullptr;
     unsigned long long* counter = nullptr;
-    unsigned char* hid = nullptr;        // batched hybrid kernel: H of problem p is an implicit identity (batched_hybrid.cuh, LAZY)
+    unsigned char* flags = nullptr;      // batched hybrid kernel: per-problem state byte (BF_* in batched_bfgs.cuh)
+    bool lazy = false;                   // batched hybrid kernel: H = I kept implicit (BF_IDENT)
+    bool derived = false;                // batched hybrid kernel: x double-buffered in x / g; g, dx, dg recomputed (BF_PARITY)
     unsigned long long* stats = nullptr; // batched hybrid kernel: running step-kind counters (HK_COUNT words)
     // large path
     double *sd = nullptr, *t = nullptr, *partial = nullptr;
@@ -155,7 +157,7 @@ static void free_handle(dzo_bfgs* o) {
     if (o->arena) { o->t = nullptr; o->d = nullptr; o->flags_t = nullptr; o->flags_d = nullptr; }   // live inside the arena
     void* ptrs[] = {o->x, o->g, o->d, o->dx, o->dg, o->H, o->f, o->L, o->iter, o->type, o->term, o->counter,
                     o->sd, o->t, o->partial, o->tile_counters, o->ctrl, o->flags_t, o->flags_d, o->done, o->arena,
-                    o->hid, o->stats};
+                    o->flags, o->stats};
     if (o->own_stream) {
         for (void* p : ptrs) {
             if (!p) continue;
@@ -225,7 +227,7 @@ static BatchedArgs batched_args(const dzo_bfgs* o, int ksteps) {
     A.iter = o->iter; A.type = o->type; A.term = o->term;
     A.f_host = o->f_host; A.term_host = o->term_host;
     A.n = (int)o->n; A.batch = o->batch; A.ksteps = ksteps; A.prefetch_rounds = g_tuning.batched_prefetch;
-    A.hid = o->hid; A.stats = o->stats;
+    A.flags = o->flags; A.lazy = o->lazy; A.derived = o->derived; A.stats = o->stats;
     A.tile = o->tile;
     return A;
 }
@@ -611,9 +613,13 @@ static int create_common(dzo_bfgs** out, int objective, int constraint, int64_t 
             return bail(rc);
         if (cudaMemsetAsync(o->stats, 0, HK_COUNT * sizeof(unsigned long long), o->stream) != cudaSuccess)
             return bail(fail(DZO_ERR_CUDA, "memset failed"));
-        // implicit identities (constructor and identity_matrix! after a GD step write no H): hybrid kernel only
-        if (objective == DZO_OBJ_ROSENBROCK && hybrid_n(n) && g_tuning.batched_lazy)
-            if ((rc = dmalloc(&o->hid, (size_t)batch))) return bail(rc);
+        if (objective == DZO_OBJ_ROSENBROCK && hybrid_n(n)) {
+            o->lazy = g_tuning.batched_lazy != 0;       // implicit identities: no H written by the constructor or after a GD step
+            // derived layout where the kernel is bound by HBM bytes; n <= 8 is bound by FP64 issue, where the recomputed
+            // gradients cost more than the bytes they save (1 M problems, n = 8: 0.320 vs 0.318 ms per launch)
+            o->derived = (g_tuning.batched_derived < 0) ? (n > 8) : (g_tuning.batched_derived != 0);
+            if ((rc = dmalloc(&o->flags, (size_t)batch))) return bail(rc);
+        }
     } else {
         const size_t nchunks = (size_t)((n + DZO_GEMV_CHUNK - 1) / DZO_GEMV_CHUNK);
         const size_t rblocks = (size_t)((o->rows + kSweepMinRows - 1) / kSweepMinRows);
@@ -785,26 +791,63 @@ static int ctrl_field(dzo_bfgs* o, T* out, F pick) {
     }
     return DZO_OK;
 }
-extern "C" {
-
-#define DZO_VEC_GETTER(name, field)                                                       \
-    int name(dzo_bfgs* o, double* out) {                                                  \
-        if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");                     \
-        return read_back(o, out, o->field, (size_t)o->n * (size_t)o->batch * 8);          \
+// derived layout: the four fields the step kernel does not store, recomputed per pair of elements from the two point
+// buffers with the operations (hence the bits) the old layout stored
+enum : int { DF_POINT = 0, DF_GRADIENT = 1, DF_DELTA_POINT = 2, DF_DELTA_GRADIENT = 3 };
+static __global__ void derived_field_kernel(BatchedArgs A, int field, double* out) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // pair t of the batch
+    const int half = A.n / 2;
+    if (t >= (long long)half * A.batch) return;
+    const long long p = t / half, e = 2 * t;
+    const unsigned fl = A.flags[p];
+    const double* cur = (fl & BF_PARITY) ? A.g : A.x;
+    const double* prev = (fl & BF_PARITY) ? A.x : A.g;
+    const double2 xc = *reinterpret_cast<const double2*>(cur + e);
+    double2 v = xc;
+    if (field == DF_GRADIENT) {
+        v = rosen_pair_grad(xc.x, xc.y);
+    } else if (field == DF_DELTA_POINT || field == DF_DELTA_GRADIENT) {
+        const bool dp = (field == DF_DELTA_POINT);
+        if (fl & BF_EXPLICIT) {
+            v = *reinterpret_cast<const double2*>((dp ? A.dx : A.dg) + e);
+        } else {
+            const double2 xp = *reinterpret_cast<const double2*>(prev + e);
+            const double2 a = dp ? xp : rosen_pair_grad(xp.x, xp.y), b = dp ? xc : rosen_pair_grad(xc.x, xc.y);
+            v = make_double2((-a.x) + b.x, (-a.y) + b.y);                  // :943-944, :949-950
+        }
     }
-DZO_VEC_GETTER(dzo_bfgs_get_point, x)
-DZO_VEC_GETTER(dzo_bfgs_get_gradient, g)
-DZO_VEC_GETTER(dzo_bfgs_get_delta_point, dx)
-DZO_VEC_GETTER(dzo_bfgs_get_delta_gradient, dg)
-DZO_VEC_GETTER(dzo_bfgs_get_direction, d)
-#undef DZO_VEC_GETTER
+    *reinterpret_cast<double2*>(out + e) = v;
+}
+static int read_vec(dzo_bfgs* o, double* out, const double* field_ptr, int derived_field) {
+    if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");
+    const size_t count = (size_t)o->n * (size_t)o->batch;
+    if (derived_field < 0 || !o->derived) return read_back(o, out, field_ptr, count * 8);
+    if (!out) return fail(DZO_ERR_INVALID_ARGUMENT, "null pointer");
+    DZO_TRY(use_device(o->device));
+    double* tmp = nullptr;
+    DZO_TRY(dmalloc_on(o->stream, &tmp, count, o->pooled));
+    const long long pairs = (long long)(count / 2);
+    derived_field_kernel<<<(unsigned)((pairs + 255) / 256), 256, 0, o->stream>>>(batched_args(o, 0), derived_field, tmp);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, tmp, count * 8, cudaMemcpyDeviceToHost, o->stream);
+    cudaFreeAsync(tmp, o->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(o->stream);
+    if (e != cudaSuccess) return fail(DZO_ERR_CUDA, "reading a derived field failed: %s", cudaGetErrorString(e));
+    return DZO_OK;
+}
+extern "C" {
+int dzo_bfgs_get_point(dzo_bfgs* o, double* out) { return read_vec(o, out, o ? o->x : nullptr, DF_POINT); }
+int dzo_bfgs_get_gradient(dzo_bfgs* o, double* out) { return read_vec(o, out, o ? o->g : nullptr, DF_GRADIENT); }
+int dzo_bfgs_get_delta_point(dzo_bfgs* o, double* out) { return read_vec(o, out, o ? o->dx : nullptr, DF_DELTA_POINT); }
+int dzo_bfgs_get_delta_gradient(dzo_bfgs* o, double* out) { return read_vec(o, out, o ? o->dg : nullptr, DF_DELTA_GRADIENT); }
+int dzo_bfgs_get_direction(dzo_bfgs* o, double* out) { return read_vec(o, out, o ? o->d : nullptr, -1); }
 
 int dzo_bfgs_get_inverse_hessian(dzo_bfgs* o, int64_t problem, double* out) {
     if (!o || problem < 0 || problem >= o->batch) return fail(DZO_ERR_INVALID_ARGUMENT, "bad arguments");
-    if (o->small && o->hid) {            // an implicit identity is materialised for the caller, not in HBM
+    if (o->small && o->lazy) {           // an implicit identity is materialised for the caller, not in HBM
         unsigned char flag = 0;
-        DZO_TRY(read_back(o, &flag, o->hid + problem, 1));
-        if (flag) {
+        DZO_TRY(read_back(o, &flag, o->flags + problem, 1));
+        if (flag & BF_IDENT) {
             for (int64_t j = 0; j < o->n; ++j)
                 for (int64_t i = 0; i < o->n; ++i) out[j * o->n + i] = (i == j) ? 1.0 : 0.0;
             return DZO_OK;
@@ -918,6 +961,13 @@ int dzo_bfgs_get_step_kind_counts(dzo_bfgs* o, int64_t* counts8, int reset) {
         DZO_CUDA(cudaMemsetAsync(o->stats, 0, sizeof c, o->stream));
         DZO_CUDA(cudaStreamSynchronize(o->stream));
     }
+    return DZO_OK;
+}
+int dzo_bfgs_batched_layout(dzo_bfgs* o, int* lazy, int* derived) {
+    if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");
+    if (!o->flags) return fail(DZO_ERR_UNSUPPORTED, "layout knobs exist for batched handles with the small-n step kernel only");
+    if (lazy) *lazy = o->lazy ? 1 : 0;
+    if (derived) *derived = o->derived ? 1 : 0;
     return DZO_OK;
 }
 int dzo_bfgs_gather_mode(dzo_bfgs* o, int* mode) {
@@ -1321,6 +1371,7 @@ int dzo_set_tuning(const char* key, int value) {
     }
     if (!strcmp(key, "batched_prefetch")) { g_tuning.batched_prefetch = value; return DZO_OK; }
     if (!strcmp(key, "batched_lazy")) { g_tuning.batched_lazy = value; return DZO_OK; }
+    if (!strcmp(key, "batched_derived")) { g_tuning.batched_derived = value; return DZO_OK; }
     return fail(DZO_ERR_INVALID_ARGUMENT, "unknown tuning key '%s'", key);
 }
 

@@ -86,6 +86,11 @@ struct Tuning {
                               // warps), 32 = always a full warp, 1..31 = forced; read when an optimizer is created
     int batched_lazy = 1;     // batched kernel: keep H = I implicit (no HBM traffic for identity_matrix!); read at create time
                               // (1M x n=16: 0.74 ms per launch with, 0.86 ms without)
+    int batched_derived = -1; // batched kernel: derived layout (batched_bfgs.cuh, BatchedArgs::derived) -- a move stores x into the
+                              // other of two point buffers and no g, dx, dg, which the getters recompute; 1 = always, 0 = every
+                              // field stored, -1 = derived for n > 8 only; read at create time.  1 M problems per launch on a
+                              // B200 (1000 W), stored -> derived ms: n = 16: 0.696 -> 0.635, n = 32: 2.39 -> 2.21, n = 8: 0.318
+                              // -> 0.320 (profiles/r03_batched_derived_ab.jsonl, DESIGN.md section 3)
 };
 extern Tuning g_tuning;
 
