@@ -551,31 +551,44 @@ class LBFGSOptimizer:
     ``LBFGSOptimizer(c_, f, g_, x0, initial_step_length, history_length)`` (:400-427); ``c_`` is ``None``
     (Julia ``nothing``) or NULL_CONSTRAINT.  Fields as in the reference: ``is_stuck`` (the live spelling of
     has_terminated), ``iteration_count``, ``current_point``, ``delta_point``, ``current_objective_value``,
-    ``delta_objective_value``, ``current_gradient``, ``delta_gradient``, ``step_direction``, ``rho_history``."""
+    ``delta_objective_value``, ``current_gradient``, ``delta_gradient``, ``step_direction``, ``rho_history``.
+
+    ``batched=True`` treats the leading axis of x0 as independent problems (README.md:12), like
+    ``BFGSOptimizer(batched=True)``: x0 has shape (batch, n), vector fields come back as (batch, n), scalar fields as
+    (batch,), ``rho_history`` as a list of ``batch`` arrays (each newest first); sums in DZO_ORDER_SEQUENTIAL."""
 
     def __init__(self, constraint_function_, objective_function, gradient_function_, initial_point,
-                 initial_step_length, history_length, device=0):
+                 initial_step_length, history_length, batched=False, device=0):
         c = NULL_CONSTRAINT if constraint_function_ is None else constraint_function_
         obj, cid = _resolve(objective_function, gradient_function_, c)
         a = np.ascontiguousarray(initial_point, dtype=np.float64)
-        if a.ndim != 1:
-            raise ValueError("initial point must be a vector")
+        if a.ndim != (2 if batched else 1):
+            raise ValueError("batched initial point must have shape (batch, n)" if batched else "initial point must be a vector")
         if not initial_step_length > 0:
             raise AssertionError("initial_step_length > 0")              # @assert :375
-        self._n = a.size
+        self._batched = bool(batched)
+        self._batch, self._n = a.shape if batched else (1, a.size)
         self._h = None
         h = C.c_void_p()
-        _check(lib().dzo_lbfgs_create(C.byref(h), obj, cid, 0, self._n, _dp(a), float(initial_step_length),
-                                      int(history_length), int(device)))
+        if batched:
+            _check(lib().dzo_lbfgs_create_batched(C.byref(h), obj, cid, 0, self._n, self._batch, _dp(a),
+                                                  float(initial_step_length), int(history_length), int(device)))
+        else:
+            _check(lib().dzo_lbfgs_create(C.byref(h), obj, cid, 0, self._n, _dp(a), float(initial_step_length),
+                                          int(history_length), int(device)))
         self._h = h
         self.history_length = int(history_length)
 
     def _vec(self, name):
-        out = np.empty(self._n)
+        out = np.empty((self._batch, self._n) if self._batched else self._n)
         _check(getattr(lib(), "dzo_lbfgs_" + name)(self._h, _dp(out)))
         return out
 
     def _sc(self, name, ctype, dtype):
+        if self._batched:
+            out = np.empty(self._batch, dtype=np.dtype(ctype))
+            _check(getattr(lib(), "dzo_lbfgs_" + name)(self._h, out.ctypes.data_as(C.POINTER(ctype))))
+            return out.astype(dtype, copy=False)
         v = ctype()
         _check(getattr(lib(), "dzo_lbfgs_" + name)(self._h, C.byref(v)))
         return np.array(v.value, dtype=dtype)
@@ -593,9 +606,17 @@ class LBFGSOptimizer:
 
     @property
     def rho_history(self):
-        cnt = C.c_int64(); rho = np.zeros(64)
-        _check(lib().dzo_lbfgs_get_rho_history(self._h, C.byref(cnt), _dp(rho)))
-        return rho[:cnt.value].copy()
+        cnt = np.zeros(self._batch, dtype=np.int64); rho = np.zeros((self._batch, 64))
+        _check(lib().dzo_lbfgs_get_rho_history(self._h, cnt.ctypes.data_as(_capi.c_i64_p), _dp(rho)))
+        if self._batched:
+            return [rho[p, :cnt[p]].copy() for p in range(self._batch)]
+        return rho[0, :cnt[0]].copy()
+
+    @property
+    def summation_order(self):
+        o = C.c_int()
+        _check(lib().dzo_lbfgs_info(self._h, None, C.byref(o), None))
+        return o.value
 
     def set_stream(self, cuda_stream):
         _check(lib().dzo_lbfgs_set_stream(self._h, C.c_void_p(cuda_stream or 0)))

@@ -117,6 +117,7 @@ def bind(lib, cpu: bool):
         sig("bfgs_get_step_kind_counts", [H, c_i64_p, I])
         sig("bfgs_batched_layout", [H, c_int_p, c_int_p])
         sig("bfgs_mirror_fields", [H, c_double_p, c_u8_p])
+        sig("lbfgs_create_batched", [HP, I, I, I64, I64, I64, c_double_p, D, I, I])
         sig("lbfgs_set_stream", [H, C.c_void_p])
         sig("lbfgs_step_async", [H, I])
         sig("lbfgs_sync", [H])

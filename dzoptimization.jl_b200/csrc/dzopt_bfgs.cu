@@ -1369,6 +1369,10 @@ int dzo_set_tuning(const char* key, int value) {
         if (value != 0 && value != 32 && value != 64 && value != 128 && value != 256) return fail(DZO_ERR_INVALID_ARGUMENT, "sweep_threads: 0, 32, 64, 128 or 256");
         g_tuning.sweep_threads = value; return DZO_OK;
     }
+    if (!strcmp(key, "lbfgs_batched_threads")) {
+        if (value != 64 && value != 128 && value != 256) return fail(DZO_ERR_INVALID_ARGUMENT, "lbfgs_batched_threads: 64, 128 or 256");
+        g_tuning.lbfgs_batched_threads = value; return DZO_OK;
+    }
     if (!strcmp(key, "batched_prefetch")) { g_tuning.batched_prefetch = value; return DZO_OK; }
     if (!strcmp(key, "batched_lazy")) { g_tuning.batched_lazy = value; return DZO_OK; }
     if (!strcmp(key, "batched_derived")) { g_tuning.batched_derived = value; return DZO_OK; }

@@ -5,6 +5,7 @@
 #include "grid_lbfgs.cuh"
 #include "legacy_lbfgs.cuh"
 #include "grid_legacy_lbfgs.cuh"
+#include "batched_lbfgs.cuh"
 
 using namespace dzo;
 
@@ -13,6 +14,9 @@ namespace dzo {
 void* grid_lbfgs_kernel_ptr(int own);
 void* grid_adgd_kernel_ptr();
 void* grid_legacy_kernel_ptr(int own);
+// the batched kernel lives in batched_lbfgs_tu.cu
+const void* batched_lbfgs_kernel_ptr(int n);
+cudaError_t batched_lbfgs_transpose(const double* src, double* dst, int n, long long batch, int to_public, cudaStream_t stream);
 }
 
 struct dzo_lbfgs {
@@ -27,12 +31,23 @@ struct dzo_lbfgs {
     int nblocks = 0, nclusters = 0;          // nclusters: CTAs of the cooperative grid
     double* part = nullptr;
     unsigned* fpart = nullptr;
+    // batch > 0: dzo_lbfgs_create_batched, one thread per problem (batched_lbfgs.cuh); every array has the batch innermost
+    // and the per-problem scalars replace ctrl
+    int64_t batch = 0;
+    int threads = 0, ctas = 0;
+    size_t smem = 0;
+    double *rho = nullptr, *f = nullptr, *df = nullptr;
+    long long* iter = nullptr;
+    int *count = nullptr, *head = nullptr;
+    unsigned char* stuck = nullptr;
+    double* scratch = nullptr;               // n x batch: the public column-major layout on its way in and out
 };
 
 static void free_lbfgs(dzo_lbfgs* o) {
     if (!o) return;
     cudaSetDevice(o->device);
-    void* ptrs[] = {o->x, o->dx, o->g, o->dg, o->d, o->S, o->Y, o->ctrl, o->part, o->fpart};
+    void* ptrs[] = {o->x, o->dx, o->g, o->dg, o->d, o->S, o->Y, o->ctrl, o->part, o->fpart,
+                    o->rho, o->f, o->df, o->iter, o->count, o->head, o->stuck, o->scratch};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (o->own_stream) cudaStreamDestroy(o->own_stream);
@@ -40,6 +55,16 @@ static void free_lbfgs(dzo_lbfgs* o) {
 }
 
 static int lbfgs_launch(dzo_lbfgs* o, int mode, int k, double L0) {
+    if (o->batch) {
+        BatchedLbfgsArgs a;
+        a.x = o->x; a.dx = o->dx; a.g = o->g; a.dg = o->dg; a.d = o->d; a.S = o->S; a.Y = o->Y; a.rho = o->rho;
+        a.f = o->f; a.df = o->df; a.iter = o->iter; a.count = o->count; a.head = o->head; a.stuck = o->stuck;
+        a.batch = o->batch; a.m = o->m; a.ksteps = k; a.mode = mode; a.initial_step_length = L0;
+        void* params[] = {&a};
+        DZO_CUDA(cudaLaunchKernel(batched_lbfgs_kernel_ptr((int)o->n), dim3((unsigned)o->ctas), dim3((unsigned)o->threads),
+                                  params, o->smem, o->stream));
+        return DZO_OK;
+    }
     if (o->use_grid) {
         GridLbfgsArgs g;
         g.x = o->x; g.dx = o->dx; g.g = o->g; g.dg = o->dg; g.d = o->d; g.S = o->S; g.Y = o->Y; g.ctrl = o->ctrl;
@@ -132,6 +157,54 @@ int dzo_lbfgs_create(dzo_lbfgs** out, int objective, int constraint, int64_t obj
     return DZO_OK;
 }
 
+int dzo_lbfgs_create_batched(dzo_lbfgs** out, int objective, int constraint, int64_t obj_param, int64_t n, int64_t batch,
+                             const double* x0, double initial_step_length, int history_length, int device) {
+    if (!out || !x0) return fail(DZO_ERR_INVALID_ARGUMENT, "null pointer");
+    *out = nullptr;
+    DZO_TRY(check_problem(objective, constraint, obj_param, n, batch));
+    if (objective != DZO_OBJ_ROSENBROCK)
+        return fail(DZO_ERR_UNSUPPORTED, "batched LBFGSOptimizer device objective: DZO_OBJ_ROSENBROCK");
+    if (n > DZO_SMALL_N_MAX) return fail(DZO_ERR_UNSUPPORTED, "batched LBFGSOptimizer needs n <= %d, got %lld", DZO_SMALL_N_MAX, (long long)n);
+    if (history_length < 1 || history_length > DZO_LBFGS_MAX_HISTORY)
+        return fail(DZO_ERR_INVALID_ARGUMENT, "history_length must be in [1, %d]", DZO_LBFGS_MAX_HISTORY);
+    if (!(initial_step_length > 0.0)) return fail(DZO_ERR_INVALID_ARGUMENT, "initial_step_length must be positive");   // :375
+    DZO_TRY(use_device(device));
+    dzo_lbfgs* o = new (std::nothrow) dzo_lbfgs();
+    if (!o) return fail(DZO_ERR_ALLOC, "out of memory");
+    o->device = device; o->n = n; o->m = history_length; o->batch = batch;
+    o->threads = g_tuning.lbfgs_batched_threads;
+    o->ctas = (int)((batch + o->threads - 1) / o->threads);
+    o->smem = (size_t)history_length * o->threads * sizeof(double);
+    auto bail = [&](int code) { free_lbfgs(o); return code; };
+    if (cudaStreamCreateWithFlags(&o->own_stream, cudaStreamNonBlocking) != cudaSuccess)
+        return bail(fail(DZO_ERR_CUDA, "cudaStreamCreate failed"));
+    o->stream = o->own_stream;
+    const size_t vb = (size_t)n * (size_t)batch * 8, hb = vb * (size_t)history_length, sb = (size_t)batch;
+    struct { void** p; size_t bytes; } allocs[] = {
+        {(void**)&o->x, vb}, {(void**)&o->dx, vb}, {(void**)&o->g, vb}, {(void**)&o->dg, vb}, {(void**)&o->d, vb},
+        {(void**)&o->scratch, vb}, {(void**)&o->S, hb}, {(void**)&o->Y, hb}, {(void**)&o->rho, sb * 8 * history_length},
+        {(void**)&o->f, sb * 8}, {(void**)&o->df, sb * 8}, {(void**)&o->iter, sb * 8}, {(void**)&o->count, sb * 4},
+        {(void**)&o->head, sb * 4}, {(void**)&o->stuck, sb}};
+    for (auto& a : allocs)
+        if (cudaMalloc(a.p, a.bytes) != cudaSuccess) {
+            cudaGetLastError();
+            return bail(fail(DZO_ERR_ALLOC, "cudaMalloc(%zu) failed", a.bytes));
+        }
+    const void* kernel = batched_lbfgs_kernel_ptr((int)n);
+    if (o->smem > 48 * 1024 &&
+        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o->smem) != cudaSuccess)
+        return bail(fail(DZO_ERR_CUDA, "the batched L-BFGS kernel cannot get %zu bytes of shared memory", o->smem));
+    if (cudaMemcpyAsync(o->scratch, x0, vb, cudaMemcpyHostToDevice, o->stream) != cudaSuccess ||
+        batched_lbfgs_transpose(o->scratch, o->x, (int)n, batch, 0, o->stream) != cudaSuccess)
+        return bail(fail(DZO_ERR_CUDA, "initial copies failed"));
+    int rc = lbfgs_launch(o, 1, 0, initial_step_length);
+    if (rc) return bail(rc);
+    if (cudaStreamSynchronize(o->stream) != cudaSuccess)
+        return bail(fail(DZO_ERR_CUDA, "constructor kernel failed: %s", cudaGetErrorString(cudaGetLastError())));
+    *out = o;
+    return DZO_OK;
+}
+
 void dzo_lbfgs_destroy(dzo_lbfgs* o) { free_lbfgs(o); }
 
 int dzo_lbfgs_set_stream(dzo_lbfgs* o, void* cuda_stream) {
@@ -165,10 +238,18 @@ static int lb_read(dzo_lbfgs* o, void* dst, const void* src, size_t bytes) {
     DZO_CUDA(cudaStreamSynchronize(o->stream));
     return DZO_OK;
 }
+// a batched handle transposes its n x batch vectors into the public column-major layout on the way out
+static int lb_read_vec(dzo_lbfgs* o, double* out, const double* field) {
+    if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");
+    if (!o->batch) return lb_read(o, out, field, (size_t)o->n * 8);
+    if (!out) return fail(DZO_ERR_INVALID_ARGUMENT, "null pointer");
+    DZO_TRY(use_device(o->device));
+    DZO_CUDA(batched_lbfgs_transpose(field, o->scratch, (int)o->n, o->batch, 1, o->stream));
+    return lb_read(o, out, o->scratch, (size_t)o->n * (size_t)o->batch * 8);
+}
 #define DZO_LB_VEC(name, field)                                                   \
     int name(dzo_lbfgs* o, double* out) {                                         \
-        if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");             \
-        return lb_read(o, out, o->field, (size_t)o->n * 8);                       \
+        return lb_read_vec(o, out, o ? o->field : nullptr);                       \
     }
 DZO_LB_VEC(dzo_lbfgs_get_point, x)
 DZO_LB_VEC(dzo_lbfgs_get_delta_point, dx)
@@ -176,29 +257,54 @@ DZO_LB_VEC(dzo_lbfgs_get_gradient, g)
 DZO_LB_VEC(dzo_lbfgs_get_delta_gradient, dg)
 DZO_LB_VEC(dzo_lbfgs_get_direction, d)
 #undef DZO_LB_VEC
-#define DZO_LB_SCALAR(name, type, expr)                                           \
+// batched handles: `batch` values straight from the per-problem array
+#define DZO_LB_SCALAR(name, type, expr, array)                                    \
     int name(dzo_lbfgs* o, type* out) {                                           \
         if (!o || !out) return fail(DZO_ERR_INVALID_ARGUMENT, "null pointer");    \
+        if (o->batch) return lb_read(o, out, o->array, (size_t)o->batch * sizeof(type)); \
         LbfgsCtrl c;                                                              \
         DZO_TRY(lb_read(o, &c, o->ctrl, sizeof c));                               \
         *out = (type)(expr);                                                      \
         return DZO_OK;                                                            \
     }
-DZO_LB_SCALAR(dzo_lbfgs_get_objective, double, c.f)
-DZO_LB_SCALAR(dzo_lbfgs_get_delta_objective, double, c.df)
-DZO_LB_SCALAR(dzo_lbfgs_get_iteration_count, int64_t, c.iter)
-DZO_LB_SCALAR(dzo_lbfgs_get_stuck, uint8_t, c.stuck != 0)
+DZO_LB_SCALAR(dzo_lbfgs_get_objective, double, c.f, f)
+DZO_LB_SCALAR(dzo_lbfgs_get_delta_objective, double, c.df, df)
+DZO_LB_SCALAR(dzo_lbfgs_get_iteration_count, int64_t, c.iter, iter)
+DZO_LB_SCALAR(dzo_lbfgs_get_stuck, uint8_t, c.stuck != 0, stuck)
 #undef DZO_LB_SCALAR
 
 int dzo_lbfgs_info(dzo_lbfgs* o, int64_t* n, int* order, int* clusters) {
     if (!o) return fail(DZO_ERR_INVALID_ARGUMENT, "null handle");
     if (n) *n = o->n;
+    if (o->batch) {
+        if (order) *order = DZO_ORDER_SEQUENTIAL;
+        if (clusters) *clusters = o->ctas;
+        return DZO_OK;
+    }
     if (order) *order = DZO_ORDER_TREE_BLOCKED;          // == DZO_ORDER_TREE for n <= DZO_TREE_BLOCK
     if (clusters) *clusters = o->use_grid ? o->nclusters : kClusterCtas;
     return DZO_OK;
 }
 int dzo_lbfgs_get_rho_history(dzo_lbfgs* o, int64_t* count, double* rho) {
     if (!o || !count || !rho) return fail(DZO_ERR_INVALID_ARGUMENT, "null pointer");
+    if (o->batch) {
+        // column p: the count[p] entries of problem p newest first, zero-padded to DZO_LBFGS_MAX_HISTORY
+        const size_t B = (size_t)o->batch;
+        double* r = new (std::nothrow) double[B * o->m];
+        int* ch = new (std::nothrow) int[2 * B];
+        if (!r || !ch) { delete[] r; delete[] ch; return fail(DZO_ERR_ALLOC, "out of memory"); }
+        int rc = lb_read(o, r, o->rho, B * o->m * 8);
+        if (!rc) rc = lb_read(o, ch, o->count, B * 4);
+        if (!rc) rc = lb_read(o, ch + B, o->head, B * 4);
+        if (!rc)
+            for (size_t p = 0; p < B; ++p) {
+                count[p] = ch[p];
+                for (int i = 0; i < DZO_LBFGS_MAX_HISTORY; ++i)
+                    rho[p * DZO_LBFGS_MAX_HISTORY + i] = (i < ch[p]) ? r[((ch[B + p] + i) % o->m) * B + p] : 0.0;
+            }
+        delete[] r; delete[] ch;
+        return rc;
+    }
     LbfgsCtrl c;
     DZO_TRY(lb_read(o, &c, o->ctrl, sizeof c));
     *count = c.count;

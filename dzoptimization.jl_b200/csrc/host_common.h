@@ -91,6 +91,8 @@ struct Tuning {
                               // field stored, -1 = derived for n > 8 only; read at create time.  1 M problems per launch on a
                               // B200 (1000 W), stored -> derived ms: n = 16: 0.696 -> 0.635, n = 32: 2.39 -> 2.21, n = 8: 0.318
                               // -> 0.320 (profiles/r03_batched_derived_ab.jsonl, DESIGN.md section 3)
+    int lbfgs_batched_threads = 128; // batched live L-BFGS (batched_lbfgs.cuh): threads per CTA, 64 / 128 / 256; read at create
+                                     // time
 };
 extern Tuning g_tuning;
 

@@ -318,6 +318,45 @@ function Base.getproperty(opt::LBFGSOptimizer, s::Symbol)
     return getfield(opt, s)
 end
 
+# `batch` independent live LBFGSOptimizers in one handle (dzo_lbfgs_create_batched, one device thread per problem, every
+# sum in the reference's sequential order); x0 is n x batch, scalar fields come back as Vectors.  (c! = NULL_CONSTRAINT)
+mutable struct BatchedLBFGSOptimizer
+    handle::Ptr{Cvoid}
+    n::Int
+    batch::Int
+    history_length::Int
+end
+function BatchedLBFGSOptimizer(c!, f, g!, x0::Matrix{Float64}, step::Float64, history_length::Int; device::Integer=0)
+    obj, cid = resolve(f, g!, c! === nothing ? NULL_CONSTRAINT : c!)
+    @assert step > 0                                                                 # :375
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:dzo_lbfgs_create_batched, libdzopt), Cint,
+        (Ref{Ptr{Cvoid}}, Cint, Cint, Int64, Int64, Int64, Ptr{Float64}, Float64, Cint, Cint),
+        h, obj, cid, 0, size(x0, 1), size(x0, 2), x0, step, history_length, device))
+    opt = BatchedLBFGSOptimizer(h[], size(x0, 1), size(x0, 2), history_length)
+    finalizer(o -> ccall((:dzo_lbfgs_destroy, libdzopt), Cvoid, (Ptr{Cvoid},), o.handle), opt)
+    return opt
+end
+function step!(opt::BatchedLBFGSOptimizer, k::Integer=1)     # k consecutive step! calls in ONE kernel launch
+    check(ccall((:dzo_lbfgs_step, libdzopt), Cint, (Ptr{Cvoid}, Cint), opt.handle, k))
+    return opt
+end
+function current_points(opt::BatchedLBFGSOptimizer)
+    out = Matrix{Float64}(undef, opt.n, opt.batch)
+    check(ccall((:dzo_lbfgs_get_point, libdzopt), Cint, (Ptr{Cvoid}, Ptr{Float64}), opt.handle, out))
+    return out
+end
+function current_objective_values(opt::BatchedLBFGSOptimizer)
+    out = Vector{Float64}(undef, opt.batch)
+    check(ccall((:dzo_lbfgs_get_objective, libdzopt), Cint, (Ptr{Cvoid}, Ptr{Float64}), opt.handle, out))
+    return out
+end
+function is_stuck_values(opt::BatchedLBFGSOptimizer)
+    out = Vector{UInt8}(undef, opt.batch)
+    check(ccall((:dzo_lbfgs_get_stuck, libdzopt), Cint, (Ptr{Cvoid}, Ptr{UInt8}), opt.handle, out))
+    return out .!= 0
+end
+
 # ================================================================== AdGDOptimizer (live src/DZOptimization.jl:179-312)
 mutable struct AdGDOptimizer
     handle::Ptr{Cvoid}
